@@ -4,6 +4,7 @@ mode, synthetic 3x32x32) on N B200s, plus p_sample-loop images/sec (bs=256) at N
 
     python bench.py [--gpus N --steps K --warmup W]           # this framework (sm_100a engine through the C ABI)
     python bench.py --impl reference [...]                     # the UNMODIFIED reference (oracle/_ref) on the host CPU
+    python bench.py [...] --dump-outputs DIR                   # + the last timed step's losses / gradients as DIR/*.npy
 
 One JSON line on stdout (rank 0).  `value` = whole-job images/s with inputs resident in HBM; `e2e` = the same step
 driven through the public Python API with the batch coming from pinned host memory and the loss read back.
@@ -128,6 +129,21 @@ def workload_config(world, B):
                         + (" + NCCL all-reduce(mean) of the flat fp32 grads, overlapped with the backward chunk by chunk" if world > 1 else ""),
             "per_gpu_batch": B, "global_batch": B * world, "resolution": "3x32x32", "parallelism": f"dp{world}",
             "l2": "4 rotating input batches; activations (2.2 GB fwd) exceed the 126 MB L2"}
+
+
+def dump_outputs(out_dir, model, losses, n_grad_sample=1 << 22):
+    """Write what the timed training step hands its caller after its last step, so that two builds can be compared output
+    for output: `losses.npy` (per-sample MSE, float32), `grad_norms.npy` (L2 norm of every parameter's gradient in
+    state_dict order, float64) and `grad_sample.npy` (float32 gradient entries at 2^22 fixed positions of the concatenated
+    parameter gradients, drawn with seed 0: all 35.7M of them would be 143 MB)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    views = model.grad_views()
+    flat = torch.cat([v.flatten() for v in views])
+    pick = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:n_grad_sample].sort().values
+    np.save(os.path.join(out_dir, "losses.npy"), losses.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_norms.npy"), torch.stack([v.double().norm() for v in views]).cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_sample.npy"), flat[pick.to(flat.device)].float().cpu().numpy())
 
 
 def reference_cpu_step(bs):
@@ -306,7 +322,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-hq", action="store_true")
     ap.add_argument("--no-stock", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's losses and gradients to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 training step")
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly ONE JSON line: anything a library writes to fd 1 meanwhile (e.g. the NCCL version banner) goes to stderr
     sys.stdout.flush()
@@ -384,6 +403,8 @@ def main():
     ms = tms.item()
     value = world * B / (ms * 1e-3)
     assert L.ddpm_device_error_flag() == 0
+    if args.dump_outputs and rank == 0:                 # before the legs below overwrite the loss and gradient buffers
+        dump_outputs(args.dump_outputs, model, losses)
     nf, nbw, npk = (__import__("ctypes").c_int() for _ in range(3))
     import ctypes as C
     L.ddpm_unet_launch_counts(h, C.byref(nf), C.byref(nbw), C.byref(npk))

@@ -21,6 +21,7 @@ from oracle import ddpm_ref as R  # noqa: E402
 def import_reference():
     """The unmodified reference, imported through oracle/ref_loader.py (matplotlib stub, SURVEY.md §8(c))."""
     from oracle import ref_loader
+    ref_loader.stage()
     return ref_loader.load()
 
 

@@ -8,8 +8,8 @@ reference's own code rather than the restatement in ``oracle/ddpm_ref.py``.
   git-ignored ``oracle/_ref/`` (listed in .gitignore, NOT in .gpurunignore, so it travels to the GPU box like a built
   ``.so``; it never enters the history).  The reference is pure Python with no ``setup.py`` / ``pyproject.toml``
   (SURVEY.md §1), so "installing" it is this copy.  Called by ``__graft_entry__.build()``.
-* ``load()``   — imports it from ``oracle/_ref`` (or straight from ``/root/reference`` when that exists and nothing was
-  staged) with the one stub the image needs: ``ddpm_torch/utils/__init__.py:1-2`` imports matplotlib, which is not
+* ``load()``   — imports it from ``oracle/_ref`` (only ``stage()`` reads the upstream checkout) with the one stub the
+  image needs: ``ddpm_torch/utils/__init__.py:1-2`` imports matplotlib, which is not
   installed (SURVEY.md §8c).  Nothing of the reference is modified.
 
 Only tests/, __graft_entry__, bench.py's reference legs and oracle/gen_golden.py may import this module.
@@ -26,29 +26,33 @@ _ITEMS = ("ddpm_torch", "ddim.py", "configs")
 
 
 def stage(src=UPSTREAM, dst=STAGED):
-    """Copy the reference's importable files into oracle/_ref (idempotent).  Returns the path, or None if src is absent."""
+    """Copy the reference's importable files into oracle/_ref (idempotent).  Returns the path, or None if src is absent.
+    Contents only, not modes: the upstream files are read-only, and a copy that kept that could not be refreshed or
+    removed by its owner."""
     if not os.path.isdir(os.path.join(src, "ddpm_torch")):
         return dst if available() else None
     os.makedirs(dst, exist_ok=True)
     for it in _ITEMS:
         s, d = os.path.join(src, it), os.path.join(dst, it)
         if os.path.isdir(s):
-            shutil.copytree(s, d, dirs_exist_ok=True, ignore=shutil.ignore_patterns("__pycache__", "*.pyc"))
+            for dirpath, dirnames, filenames in os.walk(s):
+                dirnames[:] = [n for n in dirnames if n != "__pycache__"]
+                out = os.path.join(d, os.path.relpath(dirpath, s))
+                os.makedirs(out, exist_ok=True)
+                for f in filenames:
+                    if not f.endswith(".pyc"):
+                        shutil.copyfile(os.path.join(dirpath, f), os.path.join(out, f))
         elif os.path.exists(s):
-            shutil.copy2(s, d)
+            shutil.copyfile(s, d)
     return dst
 
 
 def available():
-    return os.path.isdir(os.path.join(STAGED, "ddpm_torch")) or os.path.isdir(os.path.join(UPSTREAM, "ddpm_torch"))
+    return os.path.isdir(os.path.join(STAGED, "ddpm_torch"))
 
 
 def root():
-    if os.path.isdir(os.path.join(STAGED, "ddpm_torch")):
-        return STAGED
-    if os.path.isdir(os.path.join(UPSTREAM, "ddpm_torch")):
-        return UPSTREAM
-    return None
+    return STAGED if available() else None
 
 
 def load():

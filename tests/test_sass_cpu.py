@@ -1,5 +1,5 @@
 """The built library really is Blackwell-native code: the SASS of its hot kernels contains the tcgen05 / TMA / TMEM instructions
-(no GPU needed: cuobjdump disassembles the sm_100a cubin).  Mnemonics per /opt/skills/guides/B200_PROFILING.md:
+(no GPU needed: cuobjdump disassembles the sm_100a cubin).  Mnemonics:
 UTCHMMA = tcgen05.mma (.2CTA = cta_group::2), UTMALDG / UTMASTG = TMA load / store, LDTM = tcgen05.ld, UTCBAR = tcgen05.commit."""
 import os
 import re
@@ -11,13 +11,20 @@ import pytest
 SO = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "ddpm_torch_b200", "libddpm_b200.so")
 
 
+def _cuobjdump():
+    """cuobjdump from PATH, else from the toolkit csrc/build.sh compiles with ($NVCC, by default /usr/local/cuda/bin/nvcc)."""
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+    return shutil.which("cuobjdump") or shutil.which("cuobjdump", path=os.path.dirname(nvcc))
+
+
 @pytest.fixture(scope="module")
 def sass():
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
+    tool = _cuobjdump()
+    if tool is None:
+        pytest.skip("cuobjdump not found")
     if not os.path.exists(SO):
         pytest.fail("libddpm_b200.so is not built (python -c 'import __graft_entry__ as g; g.build()')")
-    txt = subprocess.run(["cuobjdump", "-sass", SO], capture_output=True, text=True, check=True).stdout
+    txt = subprocess.run([tool, "-sass", SO], capture_output=True, text=True, check=True).stdout
     assert "sm_100a" in txt
     per = {}
     cur = None
