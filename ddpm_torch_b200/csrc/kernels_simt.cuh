@@ -1341,83 +1341,92 @@ __global__ void k_to_uint8_nhwc(const float* __restrict__ x, unsigned char* __re
         }
     }
 }
-// out_conv on the tensor cores (unet.py:138-142): the 3x3 conv C -> CO<=4 is computed as a 1x1 GEMM to 9*CO "tap outputs"
-// per pixel, T[p][t*CO + co] = sum_c a[p][c] * w[co][c][t] (fp32, [P][32]), followed by this gather:
+// Widths of the narrow convolutions' tensor-core operands (in_conv / out_conv.2, 1..16 image channels):
+//   im2col_width(c): row length KP of a 3x3 patch matrix over c channels, 9*c columns zero padded to whole 64-wide K slabs
+//   tap_width(c):    row length TW of out_conv's tap outputs, 32 for c <= 3 (one half-slab N tile), else im2col_width(c)
+__host__ __device__ constexpr int im2col_width(int c) { return (9 * c + 63) / 64 * 64; }
+__host__ __device__ constexpr int tap_width(int c) { return c <= 3 ? 32 : im2col_width(c); }
+// out_conv on the tensor cores (unet.py:138-142): the 3x3 conv C -> CO is computed as a 1x1 GEMM to 9*CO "tap outputs"
+// per pixel, T[p][t*CO + co] = sum_c a[p][c] * w[co][c][t] (fp32, [P][TW], TW = tap_width(CO)), followed by this gather:
 // out[b][co][y][x] = bias[co] + sum_t T[(b, y + t/3 - 1, x + t%3 - 1)][t*CO + co]  (zero outside the image).
-// k_pack_tapco builds the GEMM's B operand: rows r = t*CO + co of [32][C] bf16 (rows >= 9*CO stay zero).
-__global__ void k_pack_tapco(const float* __restrict__ w /*[CO][C][9]*/, bf16* __restrict__ out /*[32][C]*/, int CO, int C) {
+// k_pack_tapco builds the GEMM's B operand: rows r = t*CO + co of [TW][C] bf16 (rows >= 9*CO stay zero).
+__global__ void k_pack_tapco(const float* __restrict__ w /*[CO][C][9]*/, bf16* __restrict__ out /*[TW][C]*/, int CO, int C) {
     pdl_entry();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= CO * C * 9) return;
     const int t = i % 9, c = (i / 9) % C, co = i / (9 * C);
     out[(long long)(t * CO + co) * C + c] = __float2bfloat16_rn(w[i]);
 }
-// transposed pack for the data gradient: out[c][t*CO + co] = w[co][c][t]   ([C][64] bf16, columns >= 9*CO stay zero)
-__global__ void k_pack_tapco_t(const float* __restrict__ w, bf16* __restrict__ out, int CO, int C) {
+// transposed pack for the data gradient: out[c][t*CO + co] = w[co][c][t]   ([C][ld] bf16, ld = im2col_width(CO), columns >= 9*CO stay zero)
+__global__ void k_pack_tapco_t(const float* __restrict__ w, bf16* __restrict__ out, int CO, int C, int ld) {
     pdl_entry();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= CO * C * 9) return;
     const int t = i % 9, c = (i / 9) % C, co = i / (9 * C);
-    out[(long long)c * 64 + t * CO + co] = __float2bfloat16_rn(w[i]);
+    out[(long long)c * ld + t * CO + co] = __float2bfloat16_rn(w[i]);
 }
-// 3x3 im2col of a narrow NCHW fp32 image (CI <= 7 channels) into NHWC bf16 rows of 64: dst[p][t*CI + ci] = src[ci][p + sign*o_t],
-// o_t = (t/3 - 1, t%3 - 1), zero outside the image and for columns >= 9*CI.  sign = +1: the conv's input patches (weight
-// gradient of in_conv); sign = -1: the patches the transposed conv sees (data and weight gradients of out_conv over d_eps).
+// 3x3 im2col of a narrow NCHW fp32 image (CI <= 16 channels) into NHWC bf16 rows of KP = im2col_width(CI):
+// dst[p][t*CI + ci] = src[ci][p + sign*o_t], o_t = (t/3 - 1, t%3 - 1), zero outside the image and for columns >= 9*CI.
+// sign = +1: the conv's input patches (in_conv forward and weight gradient); sign = -1: the patches the transposed conv sees
+// (data and weight gradients of out_conv over d_eps).  A row leaves in 16-byte pieces of 8 columns, so only one piece is held
+// in registers (a 192-wide row would not fit).
 // With qp.noise set the source is x_t = q_sample(x0, t, noise) formed on the fly (same arithmetic as k_in_conv); the centre tap
 // also stores x_t to qp.xt_out.
 template <int CI>
 __global__ void __launch_bounds__(256) k_im2col3(const float* __restrict__ src, bf16* __restrict__ dst, int B, int H, int W, int sign, const QsamplePro qp) {
     pdl_entry();
+    constexpr int KP = im2col_width(CI);
     const long long P = (long long)B * H * W;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < P; i += (long long)gridDim.x * blockDim.x) {
         const int x = (int)(i % W), y = (int)((i / W) % H); const long long b = i / ((long long)W * H);
         float qa = 1.f, qs_ = 0.f;
         if (qp.noise) { const long long tb = qp.t[b]; qa = __ldg(qp.tab_a + tb); qs_ = __ldg(qp.tab_s + tb); }
-        __align__(16) bf16 row[64];
+        uint4* o = reinterpret_cast<uint4*>(dst + i * KP);
 #pragma unroll
-        for (int j = 0; j < 64; ++j) row[j] = __float2bfloat16_rn(0.f);
+        for (int pc = 0; pc < KP / 8; ++pc) {
+            __align__(16) bf16 piece[8];
 #pragma unroll
-        for (int t = 0; t < 9; ++t) {
-            const int yy = y + sign * (t / 3 - 1), xx = x + sign * (t % 3 - 1);
-            if (yy < 0 || yy >= H || xx < 0 || xx >= W) continue;
-#pragma unroll
-            for (int ci = 0; ci < CI; ++ci) {
-                const long long j = ((b * CI + ci) * H + yy) * W + xx;
-                float v = __ldg(src + j);
-                if (qp.noise) {
-                    v = __fadd_rn(__fmul_rn(qa, v), __fmul_rn(qs_, __ldg(qp.noise + j)));
-                    if (t == 4) qp.xt_out[j] = v;
+            for (int e = 0; e < 8; ++e) {
+                const int k = pc * 8 + e, t = k / CI, ci = k % CI;
+                float v = 0.f;
+                const int yy = y + sign * (t / 3 - 1), xx = x + sign * (t % 3 - 1);
+                if (k < 9 * CI && yy >= 0 && yy < H && xx >= 0 && xx < W) {
+                    const long long j = ((b * CI + ci) * H + yy) * W + xx;
+                    v = __ldg(src + j);
+                    if (qp.noise) {
+                        v = __fadd_rn(__fmul_rn(qa, v), __fmul_rn(qs_, __ldg(qp.noise + j)));
+                        if (t == 4) qp.xt_out[j] = v;
+                    }
                 }
-                row[t * CI + ci] = __float2bfloat16_rn(v);
+                piece[e] = __float2bfloat16_rn(v);
             }
+            o[pc] = *reinterpret_cast<const uint4*>(piece);
         }
-        uint4* o = reinterpret_cast<uint4*>(dst + i * 64);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) o[j] = reinterpret_cast<const uint4*>(row)[j];
     }
 }
-// in_conv weights OIHW fp32 [Co][CI][3][3] -> bf16 [Co][64], column t*CI + ci (the patch order of k_im2col3), zero padded
-__global__ void k_pack_in(const float* __restrict__ w, bf16* __restrict__ wp, int Co, int CI) {
+// in_conv weights OIHW fp32 [Co][CI][3][3] -> bf16 [Co][KP], column t*CI + ci (the patch order of k_im2col3), zero padded
+__global__ void k_pack_in(const float* __restrict__ w, bf16* __restrict__ wp, int Co, int CI, int KP) {
     pdl_entry();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= Co * 64) return;
-    const int co = i >> 6, k = i & 63, t = k / CI, ci = k % CI;
+    if (i >= Co * KP) return;
+    const int co = i / KP, k = i % KP, t = k / CI, ci = k % CI;
     wp[i] = __float2bfloat16_rn(k < 9 * CI ? w[(co * CI + ci) * 9 + t] : 0.f);
 }
 // tap-major GEMM results back to OIHW fp32 gradients:
-//   mode 0 (out_conv):  gw[(co*C + c)*9 + t]  = S[(t*CO + co)*C + c]      S = [64][C]
-//   mode 1 (in_conv):   gw[(co*CI + ci)*9 + t] = S[co*64 + t*CI + ci]      S = [C][64]
-__global__ void k_unpack_tap(const float* __restrict__ S, float* __restrict__ gw, int CO, int CI, int mode) {
+//   mode 0 (out_conv):  gw[(co*C + c)*9 + t]  = S[(t*CO + co)*C + c]      S = [ld][C]
+//   mode 1 (in_conv):   gw[(co*CI + ci)*9 + t] = S[co*ld + t*CI + ci]     S = [C][ld]      (ld = im2col_width of the image channels)
+__global__ void k_unpack_tap(const float* __restrict__ S, float* __restrict__ gw, int CO, int CI, int mode, int ld) {
     pdl_entry();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= CO * CI * 9) return;
     const int t = i % 9, ci = (i / 9) % CI, co = i / (9 * CI);
-    gw[i] = mode == 0 ? S[(long long)(t * CO + co) * CI + ci] : S[(long long)co * 64 + t * CI + ci];
+    gw[i] = mode == 0 ? S[(long long)(t * CO + co) * CI + ci] : S[(long long)co * ld + t * CI + ci];
 }
 template <int CO>
-__global__ void __launch_bounds__(256) k_out_gather(const float* __restrict__ T /*[P][32]*/, const float* __restrict__ bias, float* __restrict__ out /*NCHW*/,
+__global__ void __launch_bounds__(256) k_out_gather(const float* __restrict__ T /*[P][TW]*/, const float* __restrict__ bias, float* __restrict__ out /*NCHW*/,
                                                    int B, int H, int W, const PsampleEpi ps) {
     pdl_entry();
+    constexpr int TW = tap_width(CO);
     const long long P = (long long)B * H * W;
     float c0 = 0.f, c1 = 0.f, c2 = 0.f, c3 = 0.f, nzsg = 0.f; uint32_t step = 0;
     if (ps.x) { c0 = ps.coef[0]; c1 = ps.coef[1]; c2 = ps.coef[2]; c3 = ps.coef[3]; nzsg = __fmul_rn(ps.coef[5], ps.coef[4]); step = (uint32_t)ps.coef[6]; }
@@ -1430,7 +1439,7 @@ __global__ void __launch_bounds__(256) k_out_gather(const float* __restrict__ T 
         for (int t = 0; t < 9; ++t) {
             const int yy = y + t / 3 - 1, xx = x + t % 3 - 1;
             if (yy < 0 || yy >= H || xx < 0 || xx >= W) continue;
-            const float* r = T + ((b * H + yy) * W + xx) * 32 + t * CO;
+            const float* r = T + ((b * H + yy) * W + xx) * TW + t * CO;
 #pragma unroll
             for (int co = 0; co < CO; ++co) acc[co] += __ldg(r + co);
         }

@@ -5,6 +5,48 @@
 
 namespace ddpm {
 
+// the narrow convolutions' per-channel-count kernels (image channels 1..16)
+inline void launch_im2col3(int ci, int nblk, cudaStream_t st, const float* src, bf16* dst, int B, int H, int W, int sign, const QsamplePro& qp) {
+    switch (ci) {
+        case 1: launch_k(k_im2col3<1>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 2: launch_k(k_im2col3<2>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 3: launch_k(k_im2col3<3>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 4: launch_k(k_im2col3<4>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 5: launch_k(k_im2col3<5>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 6: launch_k(k_im2col3<6>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 7: launch_k(k_im2col3<7>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 8: launch_k(k_im2col3<8>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 9: launch_k(k_im2col3<9>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 10: launch_k(k_im2col3<10>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 11: launch_k(k_im2col3<11>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 12: launch_k(k_im2col3<12>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 13: launch_k(k_im2col3<13>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 14: launch_k(k_im2col3<14>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        case 15: launch_k(k_im2col3<15>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+        default: launch_k(k_im2col3<16>, nblk, 256, 0, st, src, dst, B, H, W, sign, qp); break;
+    }
+}
+// (out_conv with 4 channels takes the CUDA-core k_out_conv<4>: 36 tap outputs do not fit the 32-wide route)
+inline void launch_out_gather(int co, int nblk, cudaStream_t st, const float* T, const float* bias, float* out, int B, int H, int W, const PsampleEpi& ps) {
+    switch (co) {
+        case 1: launch_k(k_out_gather<1>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 2: launch_k(k_out_gather<2>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 3: launch_k(k_out_gather<3>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 5: launch_k(k_out_gather<5>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 6: launch_k(k_out_gather<6>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 7: launch_k(k_out_gather<7>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 8: launch_k(k_out_gather<8>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 9: launch_k(k_out_gather<9>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 10: launch_k(k_out_gather<10>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 11: launch_k(k_out_gather<11>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 12: launch_k(k_out_gather<12>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 13: launch_k(k_out_gather<13>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 14: launch_k(k_out_gather<14>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        case 15: launch_k(k_out_gather<15>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+        default: launch_k(k_out_gather<16>, nblk, 256, 0, st, T, bias, out, B, H, W, ps); break;
+    }
+}
+
 // Batched matmuls of the attention block (unet.py:43-51) and their adjoints.
 //   form 0 (NT): C[b][i][j] = alpha * sum_c A[b][i][c] * B[b][j][c]     M=i, N=j, K=c
 //   form 1 (NN): C[b][i][c] = sum_j A[b][i][j] * B[b][j][c]             M=i, N=c, K=j
@@ -351,7 +393,13 @@ inline int UnetEngine::plan(int B_, int H_, int W_, bool train_, bool dry_) {
     zero_fwd_off = alloc(dry ? 0 : zf_total); zero_bwd_off = alloc(dry ? 0 : zb_total);
     const int ch = cfg.hid_channels, L = cfg.levels, nrb = cfg.num_res_blocks, E = cfg.temb_dim, Cin = cfg.in_channels, Cout = cfg.out_channels;
     if (ch % 32) return fail(-30, "hid_channels must be a multiple of 32 (GroupNorm(32))");
-    if (Cin > 4 || Cin < 1 || Cout > 4 || Cout < 1) return fail(-30, "in_channels / out_channels must be 1..4 (image channels)");
+    if (Cin > 16 || Cin < 1 || Cout > 16 || Cout < 1) return fail(-30, "in_channels / out_channels must be 1..16 (image channels)");
+    // 5..16 image channels (block-size models: C*b^2 channels at 1/b the resolution) exist only on the tensor-core routes of in_conv /
+    // out_conv.2; the CUDA-core fallbacks stop at 4
+    const bool wide_in = Cin > 4, wide_out = Cout > 4;
+    if ((wide_in || wide_out) && !(ch % 64 == 0 && tc_ok_geom(H, W)))
+        return fail(-30, "in_channels / out_channels of 5..16 need the tensor-core narrow convolutions: hid_channels %% 64 == 0 "
+                         "and a tensor-core resolution (got hid_channels=%d, %dx%d)", ch, H, W);
     if ((H >> (L - 1)) < 1 || (H % (1 << (L - 1))) || (W % (1 << (L - 1)))) return fail(-30, "resolution not divisible by 2^(levels-1)");
     UnetEngine* self = this;
 
@@ -537,29 +585,26 @@ inline int UnetEngine::plan(int B_, int H_, int W_, bool train_, bool dry_) {
         // h0 feeds the first norm1 and (as the last skip) the final up block's norm1: its statistics come out of this kernel
         double* qs0 = nullptr;
         if (ch % 32 == 0 && (H * W) % 32 == 0 && !getenv("DDPM_NO_GN_EPI")) { h0.qs = (long long)zero_fwd((size_t)B * (ch / 4) * 2 * 8); qs0 = at<double>((size_t)h0.qs); }
-        // tensor-core route: X = im2col(x) [P][64] bf16 (27 patch columns, zero padded to one K slab) and a 1x1 "conv" over it;
-        // the training backward reuses X for the weight gradient.  (CUDA-core k_in_conv otherwise.)
+        // tensor-core route: X = im2col(x) [P][KP] bf16 (9*Cin patch columns, zero padded to whole K slabs: KP = 64 up to 7
+        // channels, 128 / 192 for 8..16) and a 1x1 "conv" over it; the training backward reuses X for the weight gradient.
+        // (CUDA-core k_in_conv otherwise, up to 4 channels.)
         static const bool no_tc_inconv = getenv("DDPM_NO_TC_INCONV") != nullptr;
-        const bool tc_in = !no_tc_inconv && ch % 64 == 0 && tc_ok_geom(H, W) && 9 * Cin <= 64 && Cin <= 4;
+        const bool tc_in = wide_in || (!no_tc_inconv && ch % 64 == 0 && tc_ok_geom(H, W) && Cin <= 4);
+        const int KP = im2col_width(Cin);
         T4 Xcol;
         if (tc_in) {
-            Xcol = newT(B, H, W, 64);
+            Xcol = newT(B, H, W, KP);
             bf16* Xp = bp(Xcol);
-            bf16* wpk = at<bf16>(alloc((size_t)ch * 64 * 2));
-            const int npk = (ch * 64 + 255) / 256; const int chn = ch, cin = Cin;
-            push(pack_ops, "in_conv.pack", 0, [=](cudaStream_t st) { launch_k(k_pack_in, npk, 256, 0, st, wi, wpk, chn, cin); return (int)cudaGetLastError(); });
+            bf16* wpk = at<bf16>(alloc((size_t)ch * KP * 2));
+            const int npk = (ch * KP + 255) / 256; const int chn = ch, cin = Cin;
+            push(pack_ops, "in_conv.pack", 0, [=](cudaStream_t st) { launch_k(k_pack_in, npk, 256, 0, st, wi, wpk, chn, cin, KP); return (int)cudaGetLastError(); });
             pack_ops.back().wait_pack = 1;             // "early" pack: in_conv is the first consumer of the forward pass
             const int nim = grid_for((long long)B * H * W);
             push(fwd_ops, "in_conv.im2col", 0, [=](cudaStream_t st) {
-                const QsamplePro qp = self->qs_pro;   // training: x_t = q_sample(x0, t, noise) is formed while the patches are gathered
-                switch (cin) {
-                    case 1: launch_k(k_im2col3<1>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, qp); break;
-                    case 2: launch_k(k_im2col3<2>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, qp); break;
-                    case 3: launch_k(k_im2col3<3>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, qp); break;
-                    default: launch_k(k_im2col3<4>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, qp); break;
-                }
+                // training: x_t = q_sample(x0, t, noise) is formed while the patches are gathered
+                launch_im2col3(cin, nim, st, self->x_in, Xp, Bn, Hn, Wn, 1, self->qs_pro);
                 return (int)cudaGetLastError(); });
-            ConvSpec c; c.name = "in_conv"; c.in = one(Xcol); c.ksize = 1; c.wp = wpk; c.ldw = 64; c.bias = bi; c.out = h0; c.Co = ch; c.Ho = H; c.Wo = W;
+            ConvSpec c; c.name = "in_conv"; c.in = one(Xcol); c.ksize = 1; c.wp = wpk; c.ldw = KP; c.bias = bi; c.out = h0; c.Co = ch; c.Ho = H; c.Wo = W;
             c.want_qstats = true;
             const size_t first_conv = fwd_ops.size();
             h0.qs = conv_op(fwd_ops, c, nullptr);
@@ -583,24 +628,18 @@ inline int UnetEngine::plan(int B_, int H_, int W_, bool train_, bool dry_) {
             bwd_flops += 2.0 * P * ch * Cin * 9;
             const long long s_c = (long long)Cin * 9;
             static const bool no_tc_in = getenv("DDPM_NO_TC_OUTCONV") != nullptr;
-            if (!no_tc_in && ch % 64 == 0 && tc_ok_geom(H, W) && 9 * Cin <= 64) {
-                // weight gradient on the tensor cores: X = im2col(x) [P][64] bf16, S[ch][64] = dY^T x X (MN-major GEMM, side stream)
-                T4 X = tc_in ? Xcol : newT(B, H, W, 64);
+            if (wide_in || (!no_tc_in && ch % 64 == 0 && tc_ok_geom(H, W) && 9 * Cin <= 64)) {
+                // weight gradient on the tensor cores: X = im2col(x) [P][KP] bf16, S[ch][KP] = dY^T x X (MN-major GEMM, side stream)
+                T4 X = tc_in ? Xcol : newT(B, H, W, KP);
                 bf16* Xp = bp(X);
                 const int nim = grid_for(P);
                 if (!tc_in) push(bwd_ops, "in_conv.im2col", 0, [=](cudaStream_t st) {
-                    const QsamplePro q0{nullptr, nullptr, nullptr, nullptr, nullptr};
-                    switch (Cin) {
-                        case 1: launch_k(k_im2col3<1>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, q0); break;
-                        case 2: launch_k(k_im2col3<2>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, q0); break;
-                        case 3: launch_k(k_im2col3<3>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, q0); break;
-                        default: launch_k(k_im2col3<4>, nim, 256, 0, st, self->x_in, Xp, Bn, Hn, Wn, 1, q0); break;
-                    }
+                    launch_im2col3(Cin, nim, st, self->x_in, Xp, Bn, Hn, Wn, 1, QsamplePro{nullptr, nullptr, nullptr, nullptr, nullptr});
                     return (int)cudaGetLastError(); }, 1, true);
-                float* S2 = at<float>(zero_bwd((size_t)ch * 64 * 4));
+                float* S2 = at<float>(zero_bwd((size_t)ch * KP * 4));
                 wgrad_op("in_conv.wgrad", dY, one(X), 1, 1, MAP_NORMAL, S2, ch);
                 const int nun = (ch * Cin * 9 + 255) / 256;
-                push(bwd_ops, "in_conv.wunpack", 0, [=](cudaStream_t st) { launch_k(k_unpack_tap, nun, 256, 0, st, S2, gw, ch, Cin, 1); return (int)cudaGetLastError(); }, 1, true);
+                push(bwd_ops, "in_conv.wunpack", 0, [=](cudaStream_t st) { launch_k(k_unpack_tap, nun, 256, 0, st, S2, gw, ch, Cin, 1, KP); return (int)cudaGetLastError(); }, 1, true);
                 colsum_op("in_conv.bias", dY, nullptr, 0, gb, nullptr, ch);
                 return;
             }
@@ -644,7 +683,7 @@ inline int UnetEngine::plan(int B_, int H_, int W_, bool train_, bool dry_) {
         if (i != 0) h = up_conv(p + "." + std::to_string(nrb + 1) + ".1", h);
     }
     if (blk != nblocks) return fail(-31, "internal: block count mismatch %d vs %d", blk, nblocks);
-    // ---- out_conv (unet.py:138-142,232): GN -> SiLU -> conv3x3 (C -> Cout<=4) -> NCHW fp32
+    // ---- out_conv (unet.py:138-142,232): GN -> SiLU -> conv3x3 (C -> Cout<=16) -> NCHW fp32
     cur_tag = "u" + std::to_string(L - 1);           // its parameters sit right behind upsamples.level_{L-1} in the flat buffer
     {
         if (ch > 256) return fail(-30, "hid_channels > 256 unsupported by the narrow out_conv kernels");
@@ -658,25 +697,27 @@ inline int UnetEngine::plan(int B_, int H_, int W_, bool train_, bool dry_) {
         const double fl = 2.0 * B * H * W * ch * Cout * 9;
         fwd_flops += fl;
         static const bool no_tc_out = getenv("DDPM_NO_TC_OUTCONV") != nullptr;
-        bool tc_out = !no_tc_out && ch % 64 == 0 && tc_ok_geom(H, W) && 9 * Cout <= 32;
+        bool tc_out = wide_out || (!no_tc_out && ch % 64 == 0 && tc_ok_geom(H, W) && 9 * Cout <= 32);
+        // tap-output width of the forward GEMM (32 up to 3 channels, 64 / 128 / 192 for 5..16) and patch width of the backward's im2col
+        const int TW = tap_width(Cout), KPo = im2col_width(Cout);
         bf16* w27t = nullptr;
         if (tc_out) {
-            // tensor-core path: 1x1 GEMM a[P][ch] x W27[32][ch]^T -> fp32 tap outputs T[P][32], then a 9-point gather
-            bf16* w27 = at<bf16>(alloc_once_zero((size_t)32 * ch * 2));
-            float* T = at<float>(alloc((size_t)B * H * W * 32 * 4));
+            // tensor-core path: 1x1 GEMM a[P][ch] x W27[TW][ch]^T -> fp32 tap outputs T[P][TW], then a 9-point gather
+            bf16* w27 = at<bf16>(alloc_once_zero((size_t)TW * ch * 2));
+            float* T = at<float>(alloc((size_t)B * H * W * TW * 4));
             const int npk = (Cout * ch * 9 + 255) / 256;
             push(pack_ops, "out_conv.pack27", 0, [=](cudaStream_t st) { launch_k(k_pack_tapco, npk, 256, 0, st, wo, w27, Cout, ch); return (int)cudaGetLastError(); });
             if (train) {
-                w27t = at<bf16>(alloc_once_zero((size_t)ch * 64 * 2));
+                w27t = at<bf16>(alloc_once_zero((size_t)ch * KPo * 2));
                 bf16* w27tp = w27t;
-                push(pack_ops, "out_conv.pack27t", 0, [=](cudaStream_t st) { launch_k(k_pack_tapco_t, npk, 256, 0, st, wo, w27tp, Cout, ch); return (int)cudaGetLastError(); });
+                push(pack_ops, "out_conv.pack27t", 0, [=](cudaStream_t st) { launch_k(k_pack_tapco_t, npk, 256, 0, st, wo, w27tp, Cout, ch, KPo); return (int)cudaGetLastError(); });
             }
             ddpm_gemm_desc d; memset(&d, 0, sizeof d);
-            d.mode = GEMM_KK; d.M = B * H * W; d.N = 32; d.block_n = 64; d.W = W; d.H = H; d.NB = B;
+            d.mode = GEMM_KK; d.M = B * H * W; d.N = TW; d.block_n = 64; d.W = W; d.H = H; d.NB = B;
             d.a_ptr[0] = ap; d.a_C[0] = ch; d.a_ld[0] = ch;
             d.nseg = 1; d.seg_map[0] = 0; d.seg_taps[0] = 1; d.seg_kchunks[0] = ch / 64; d.seg_cbase[0] = 0;
-            d.b_ptr = w27; d.b_K = ch; d.b_rows = 32; d.b_batch = 1; d.b_ld = ch; d.b_bs = 0;
-            d.out = T; d.ldo = 32; d.alpha = 1.f; d.grid_z = 1; d.flags = EPI_OUT_F32;
+            d.b_ptr = w27; d.b_K = ch; d.b_rows = TW; d.b_batch = 1; d.b_ld = ch; d.b_bs = 0;
+            d.out = T; d.ldo = TW; d.alpha = 1.f; d.grid_z = 1; d.flags = EPI_OUT_F32;
             ++n_tc_gemms;
             if (!dry) {
                 GemmLaunch g; const int rc = build_gemm(d, g);
@@ -685,11 +726,7 @@ inline int UnetEngine::plan(int B_, int H_, int W_, bool train_, bool dry_) {
             } else push(fwd_ops, "out_conv.2", fl, [](cudaStream_t) { return 0; });
             gather_fused_tail = true;             // the sampler's alpha/beta update rides in this kernel (ddpm_sampler_step)
             push(fwd_ops, "out_conv.2.gather", 0, [=](cudaStream_t st) {
-                switch (Cout) {
-                    case 1: launch_k(k_out_gather<1>, nblk, 256, 0, st, T, bo, self->eps_dst, Bn, Hn, Wn, self->ps_epi); break;
-                    case 2: launch_k(k_out_gather<2>, nblk, 256, 0, st, T, bo, self->eps_dst, Bn, Hn, Wn, self->ps_epi); break;
-                    default: launch_k(k_out_gather<3>, nblk, 256, 0, st, T, bo, self->eps_dst, Bn, Hn, Wn, self->ps_epi); break;
-                }
+                launch_out_gather(Cout, nblk, st, T, bo, self->eps_dst, Bn, Hn, Wn, self->ps_epi);
                 return (int)cudaGetLastError(); });
         } else
         push(fwd_ops, "out_conv.2", fl, [=](cudaStream_t st) {
@@ -712,27 +749,23 @@ inline int UnetEngine::plan(int B_, int H_, int W_, bool train_, bool dry_) {
                 const long long P = (long long)Bn * Hn * Wn; const int ppb = 256; const int nb = (int)((P + ppb - 1) / ppb);
                 bwd_flops += 2.0 * fl;
                 if (tc_out) {
-                    // tensor-core backward: E = im2col(d_eps) [P][64] bf16 (shared by both gradients);
-                    // d_a = E x W27^T (1x1 conv 64 -> ch), dW = E^T x a (MN-major GEMM on the side stream) -> OIHW
-                    T4 E = newT(B, H, W, 64);
+                    // tensor-core backward: E = im2col(d_eps) [P][KPo] bf16 (shared by both gradients);
+                    // d_a = E x W27^T (1x1 conv KPo -> ch), dW = E^T x a (MN-major GEMM on the side stream) -> OIHW
+                    T4 E = newT(B, H, W, KPo);
                     bf16* Ep = bp(E);
                     const int nim = grid_for((long long)Bn * Hn * Wn);
                     push(bwd_ops, "out_conv.2.im2col", 0, [=](cudaStream_t st) {
                         const float* de = self->deps_src;
                         launch_k(k_chansum_nchw, dim3(64, Cout), 256, 0, st, de, gb, Bn, Cout, Hn * Wn);
-                        switch (Cout) {
-                            case 1: launch_k(k_im2col3<1>, nim, 256, 0, st, de, Ep, Bn, Hn, Wn, -1, QsamplePro{nullptr, nullptr, nullptr, nullptr, nullptr}); break;
-                            case 2: launch_k(k_im2col3<2>, nim, 256, 0, st, de, Ep, Bn, Hn, Wn, -1, QsamplePro{nullptr, nullptr, nullptr, nullptr, nullptr}); break;
-                            default: launch_k(k_im2col3<3>, nim, 256, 0, st, de, Ep, Bn, Hn, Wn, -1, QsamplePro{nullptr, nullptr, nullptr, nullptr, nullptr}); break;
-                        }
+                        launch_im2col3(Cout, nim, st, de, Ep, Bn, Hn, Wn, -1, QsamplePro{nullptr, nullptr, nullptr, nullptr, nullptr});
                         return (int)cudaGetLastError(); }, 2);
-                    ConvSpec cs; cs.name = "out_conv.2.dgrad"; cs.in = one(E); cs.ksize = 1; cs.wp = w27t; cs.ldw = 64;
+                    ConvSpec cs; cs.name = "out_conv.2.dgrad"; cs.in = one(E); cs.ksize = 1; cs.wp = w27t; cs.ldw = KPo;
                     cs.out = d_a; cs.Co = ch; cs.Ho = H; cs.Wo = W;
                     conv_op(bwd_ops, cs, nullptr);
-                    float* S = at<float>(zero_bwd((size_t)64 * ch * 4));
-                    wgrad_op("out_conv.2.wgrad", E, one(a_out), 1, 1, MAP_NORMAL, S, 64);
+                    float* S = at<float>(zero_bwd((size_t)KPo * ch * 4));
+                    wgrad_op("out_conv.2.wgrad", E, one(a_out), 1, 1, MAP_NORMAL, S, KPo);
                     const int nun = (Cout * ch * 9 + 255) / 256;
-                    push(bwd_ops, "out_conv.2.wunpack", 0, [=](cudaStream_t st) { launch_k(k_unpack_tap, nun, 256, 0, st, S, gw, Cout, ch, 0); return (int)cudaGetLastError(); }, 1, true);
+                    push(bwd_ops, "out_conv.2.wunpack", 0, [=](cudaStream_t st) { launch_k(k_unpack_tap, nun, 256, 0, st, S, gw, Cout, ch, 0, KPo); return (int)cudaGetLastError(); }, 1, true);
                 } else
                 push(bwd_ops, "out_conv.2.bwd", 2.0 * fl, [=](cudaStream_t st) {
                     const float* de = self->deps_src;

@@ -9,13 +9,17 @@ the configuration is the one every reference config uses (eps-prediction, fixed 
 * ``p_sample`` / ``p_sample_step`` -> the engine's sampler step (UNet forward + the alpha/beta update of
   diffusion.py:107-158 in one launch sequence, replayed from a CUDA graph once per timestep).
 
-Any other ``denoise_fn`` (toy MLPs, wrappers) takes the generic formulas below, written with plain torch ops.
+A block-size model (train.py:63-73: ``ModelWrapper(UNet(C*b*b, ...), PixelUnshuffle(b), PixelShuffle(b))``, optionally inside
+DDP) takes the same native paths on the inner layout [B, C*b*b, H/b, W/b]; the pixel (un)shuffles are torch copies around them.
+Any other ``denoise_fn`` (toy MLPs, other wrappers) takes the generic formulas below, written with plain torch ops.
 """
 import ctypes as C
 
 import math
 
 import torch
+import torch.nn as nn
+import torch.nn.functional as F
 
 from . import _lib
 from .unet import UNet
@@ -43,15 +47,38 @@ def get_beta_schedule(beta_schedule, beta_start, beta_end, timesteps, dtype=torc
 
 
 def _native(denoise_fn):
-    """Unwrap DDP / holders; return the engine-backed UNet or None."""
+    """Unwrap DDP / holders and a pixel (un)shuffle model wrapper (utils/train.py:349-367); return (engine UNet, block size b)
+    or (None, 1).  A wrapper counts only when its transforms are exactly PixelUnshuffle(b) / PixelShuffle(b) with the same b
+    around an engine UNet: the native paths then run the UNet on pixel_unshuffle(x, b) and shuffle its output back."""
     m = denoise_fn
     for _ in range(3):
         if isinstance(m, UNet):
-            return m
+            return m, 1
+        pre, post = getattr(m, "pre_transform", None), getattr(m, "post_transform", None)
+        if hasattr(m, "_model") and type(pre) is nn.PixelUnshuffle and type(post) is nn.PixelShuffle:
+            inner = m._model
+            if pre.downscale_factor == post.upscale_factor and isinstance(inner, UNet):
+                return inner, pre.downscale_factor
+            return None, 1
         m = getattr(m, "module", None)
         if m is None:
-            return None
-    return None
+            return None, 1
+    return None, 1
+
+
+def _to_inner(x, model, b):
+    """pixel_unshuffle(x, b) as a contiguous fp32 batch for the engine UNet of a block-size model, whose plan reads exactly
+    model.in_channels channels."""
+    if x.shape[1] * b * b != model.in_channels:
+        raise ValueError(f"block size {b}: the UNet takes {model.in_channels} channels, the batch has {x.shape[1]}")
+    return F.pixel_unshuffle(x.float(), b).contiguous()
+
+
+def _unshuffle_into(dst, src, b):
+    """dst[B, C*b*b, H/b, W/b] = pixel_unshuffle(src[B, C, H, W], b) as one copy into an existing buffer (no allocation, so it can
+    sit inside a captured graph)."""
+    B, Cc, H, W = src.shape
+    dst.view(B, Cc, b, b, H // b, W // b).copy_(src.view(B, Cc, H // b, b, W // b, b).permute(0, 1, 3, 5, 2, 4))
 
 
 def _flat_mean(x):
@@ -163,9 +190,10 @@ class GaussianDiffusion:
         return (model_mean, model_var, model_logvar, pred_x_0) if return_pred else (model_mean, model_var, model_logvar)
 
     def _fast_ok(self, denoise_fn):
-        m = _native(denoise_fn)
+        """(engine UNet, block size) when the native paths apply, else (None, 1)."""
+        m, b = _native(denoise_fn)
         ok = m is not None and self.model_mean_type == "eps" and self.model_var_type in ("fixed-small", "fixed-large")
-        return m if ok else None
+        return (m, b) if ok else (None, 1)
 
     # ------------------------------------------------------------------ sampling
     def p_sample_step(self, denoise_fn, x_t, t, clip_denoised=True, return_pred=False, generator=None):
@@ -191,7 +219,7 @@ class GaussianDiffusion:
     def p_sample(self, denoise_fn, shape=None, device=torch.device("cpu"), noise=None, seed=None, rng="torch", use_graph=True, split=None):
         """diffusion.py:160-174.  ``rng="torch"`` consumes a torch.Generator exactly like the reference (bit-identical
         noise stream); ``rng="philox"`` draws the per-step noise inside the step kernel (one launch sequence per step)."""
-        model = self._fast_ok(denoise_fn)
+        model, blk = self._fast_ok(denoise_fn)
         B = (shape or noise.shape)[0]
         gen = torch.Generator(device).manual_seed(seed) if seed is not None else None
         x_t = torch.empty(shape, device=device).normal_(generator=gen) if noise is None else noise.to(device)
@@ -203,6 +231,8 @@ class GaussianDiffusion:
                 t.fill_(ti)
                 x_t = self.p_sample_step(fn, x_t, t, generator=gen)
             return x_t
+        if blk > 1:        # x_T is drawn in the outer shape, as the reference does, and the chain runs on the UNet's layout
+            return F.pixel_shuffle(_native_sample_loop(self, model, _to_inner(x_t, model, blk), gen, rng, seed, use_graph, split, blk), blk)
         return _native_sample_loop(self, model, x_t.contiguous().float().clone(), gen, rng, seed, use_graph, split)
 
     def _wrap_denoise(self, denoise_fn, device):
@@ -218,11 +248,12 @@ class GaussianDiffusion:
         n = self.timesteps // pred_freq
         preds = torch.zeros((n, B) + tuple(shape[1:]), dtype=torch.float32)
         idx = n
-        model = self._fast_ok(denoise_fn)
+        model, blk = self._fast_ok(denoise_fn)
         if model is not None and x_t.is_cuda:
             L = _lib.lib()
             dev = model.flat_params.device
-            x_t = x_t.contiguous().float().clone()
+            x_out = x_t
+            x_t = _to_inner(x_t, model, blk) if blk > 1 else x_t.contiguous().float().clone()
             _, _, H, W = x_t.shape
             was_training = model.training
             model.eval()
@@ -233,16 +264,19 @@ class GaussianDiffusion:
                     _lib.check(L.ddpm_sampler_setup(h, coef.shape[0], tmod.data_ptr(), coef.data_ptr()), "sampler_setup")
                     _lib.check(L.ddpm_sampler_reset(h, self.timesteps - 1, _lib.stream_ptr(dev)), "sampler_reset")
                     z, pred = torch.empty_like(x_t), torch.empty_like(x_t)
+                    z_out = torch.empty_like(x_out) if blk > 1 else z      # noise is drawn in the outer shape (diffusion.py:155)
                     for ti in range(self.timesteps - 1, -1, -1):
-                        z.normal_(generator=gen)
+                        z_out.normal_(generator=gen)
+                        if blk > 1:
+                            _unshuffle_into(z, z_out, blk)
                         _lib.check(L.ddpm_sampler_step_pred(h, x_t.data_ptr(), z.data_ptr(), 0, pred.data_ptr(), _lib.stream_ptr(dev)), "sampler_step")
                         if (ti + 1) % pred_freq == 0:
                             idx -= 1
-                            preds[idx] = pred.cpu()
+                            preds[idx] = (F.pixel_shuffle(pred, blk) if blk > 1 else pred).cpu()
             finally:
                 if was_training:
                     model.train()
-            return x_t.cpu(), preds
+            return (F.pixel_shuffle(x_t, blk) if blk > 1 else x_t).cpu(), preds
         t = torch.empty(B, dtype=torch.int64, device=device)
         fn = self._wrap_denoise(denoise_fn, device)
         for ti in range(self.timesteps - 1, -1, -1):
@@ -257,8 +291,12 @@ class GaussianDiffusion:
     def train_losses(self, denoise_fn, x_0, t, noise=None):
         if noise is None:
             noise = torch.randn_like(x_0)
-        model = self._fast_ok(denoise_fn)
+        model, blk = self._fast_ok(denoise_fn)
         if model is not None and self.loss_type == "mse" and x_0.is_cuda:
+            if blk > 1:
+                # q_sample is elementwise and the per-sample mean is invariant under the pixel permutation: the fused loss on the
+                # unshuffled batch is the reference's loss of the wrapped model
+                x_0, noise = _to_inner(x_0, model, blk), _to_inner(noise, model, blk)
             return _TrainLossFn.apply(self, model, denoise_fn, x_0.contiguous().float(), t.contiguous(), noise.contiguous().float(),
                                       *model._params)
         x_t = self.q_sample(x_0, t, noise=noise)
@@ -368,9 +406,12 @@ def _ddp_allreduce(wrapper, model):
     allreduce_grads_overlapped_(model, group=getattr(wrapper, "process_group", None))     # chunk-wise, overlapped with the backward's tail
 
 
-def _native_sample_loop(diffusion, model, x, gen, rng, seed, use_graph, split=None):
+def _native_sample_loop(diffusion, model, x, gen, rng, seed, use_graph, split=None, blk=1):
     """T sampler steps on the engine: per step {noise draw, step-table fetch, UNet forward with the alpha/beta update in the final
     conv's epilogue}; captured once, replayed T times - one graph launch per timestep.
+
+    ``blk > 1`` (block-size model): ``x`` is already in the UNet's layout [B, C*b*b, H/b, W/b]; each step's torch noise is drawn in
+    the outer shape [B, C, H, W] and unshuffled into the step's noise buffer, so the stream is the reference's draw for draw.
 
     ``split=2`` (opt-in; DDPM_SAMPLER_SPLIT overrides the default of 1 - measured on B200 at bs=256: 5.46 vs 5.47 ms per step, no gain, since half-batch kernels are less efficient): the batch is cut into two
     halves with their own plans, run on two forked streams inside the SAME captured graph, so that one half's HBM-bound
@@ -392,14 +433,14 @@ def _native_sample_loop(diffusion, model, x, gen, rng, seed, use_graph, split=No
     ctx_dev = torch.cuda.device(dev)
     ctx_dev.__enter__()          # every launch below targets the model's device (generate.py:59 never calls set_device)
     try:
-        return _native_sample_loop_on_device(diffusion, model, x, gen, rng, seed, use_graph, split, Bh, H, W, was_training)
+        return _native_sample_loop_on_device(diffusion, model, x, gen, rng, seed, use_graph, split, Bh, H, W, was_training, blk)
     finally:
         ctx_dev.__exit__(None, None, None)
         if was_training:
             model.train()
 
 
-def _native_sample_loop_on_device(diffusion, model, x, gen, rng, seed, use_graph, split, Bh, H, W, was_training):
+def _native_sample_loop_on_device(diffusion, model, x, gen, rng, seed, use_graph, split, Bh, H, W, was_training, blk=1):
     L = _lib.lib()
     # weights are re-packed unconditionally at the head of every loop: the reference EMA swaps values with `p.data.copy_`
     # (utils/train.py:307-316), which no version counter sees; 0.2 ms against a T-step loop
@@ -412,15 +453,18 @@ def _native_sample_loop_on_device(diffusion, model, x, gen, rng, seed, use_graph
     # p_sample once per batch, and re-capturing ~150 kernels per call costs more than a dozen DDIM steps.  A cached graph owns
     # persistent x / z buffers and (for seeded runs) a persistent registered generator that takes over the caller's generator state.
     ent = None
+    B, Cc = x.shape[:2]
+    outer = (B, Cc // (blk * blk), H * blk, W * blk)
     if use_graph and rng == "torch" and S > 1:
-        key = (x.shape, split, S, gen is not None, model._plan_epoch, tuple(model._aux[i].get("epoch", 0) for i in range(1, split)))
+        key = (x.shape, blk, split, S, gen is not None, model._plan_epoch, tuple(model._aux[i].get("epoch", 0) for i in range(1, split)))
         ent = model._sampler_cache.get(key)
         if ent is None:
             if len(model._sampler_cache) >= 4:
                 model._sampler_cache.clear()
             ent = model._sampler_cache[key] = {"x": torch.empty_like(x), "z": torch.empty_like(x), "graph": None,
+                                               "z_out": x.new_empty(outer) if blk > 1 else None,
                                                "gen": torch.Generator(x.device) if gen is not None else None}
-        xb, z = ent["x"], ent["z"]
+        xb, z, z_out = ent["x"], ent["z"], ent["z_out"]
         xb.copy_(x)
         x = xb
         if gen is not None:
@@ -428,6 +472,7 @@ def _native_sample_loop_on_device(diffusion, model, x, gen, rng, seed, use_graph
             gen = ent["gen"]
     else:
         z = torch.empty_like(x) if rng == "torch" else None
+        z_out = x.new_empty(outer) if (rng == "torch" and blk > 1) else None
     stream = torch.cuda.current_stream()
     for h in hs:
         _lib.check(L.ddpm_sampler_setup(h, S, tmod.data_ptr(), coef.data_ptr()), "sampler_setup")
@@ -450,7 +495,10 @@ def _native_sample_loop_on_device(diffusion, model, x, gen, rng, seed, use_graph
             cur.wait_stream(s_)
 
     def draw():
-        if z is not None:
+        if z_out is not None:                   # block-size model: the reference draws in the outer shape
+            z_out.normal_(generator=gen)
+            _unshuffle_into(z, z_out, blk)
+        elif z is not None:
             z.normal_(generator=gen)            # diffusion.py:155 - the reference's stream, drawn on the device
 
     def capture():

@@ -303,8 +303,9 @@ class _UNetFn(torch.autograd.Function):
 
 class ModelWrapper(nn.Module):
     """utils/train.py:349-367: optional pre / post transforms around a model (the reference uses PixelUnshuffle / PixelShuffle
-    when ``block_size > 1``, train.py:70-73).  A wrapped model is a NON-native ``denoise_fn`` for the diffusion classes: the
-    loop and the loss run through the generic torch formulas while the inner ``UNet`` still executes on the engine."""
+    when ``block_size > 1``, train.py:70-73).  ``ModelWrapper(UNet(C*b*b, ...), nn.PixelUnshuffle(b), nn.PixelShuffle(b))`` (also
+    inside DDP) takes the diffusion classes' native training and sampling paths on the unshuffled layout; with any other
+    transforms the wrapper is a generic ``denoise_fn`` (torch formulas, the inner ``UNet`` still executes on the engine)."""
 
     def __init__(self, model, pre_transform=None, post_transform=None):
         super().__init__()

@@ -108,6 +108,8 @@ int ddpm_attn_fused_bwd_run(const void* qkv, const void* d_out, const void* prob
  */
 typedef struct ddpm_unet_cfg {          /* mirrors UNet(in_channels, hid_channels, out_channels, ch_multipliers,   */
     int in_channels, hid_channels, out_channels;   /* num_res_blocks, apply_attn, time_embedding_dim, drop_rate)  unet.py:96-107 */
+    /* in_channels / out_channels: 1..16 image channels (C*b*b of a block-size model); 5..16 need hid_channels % 64 == 0 and a
+     * tensor-core resolution, otherwise ddpm_unet_workspace_bytes / ddpm_unet_plan return an error */
     int levels; int ch_mult[8];
     int num_res_blocks; int attn[8];
     int temb_dim;                       /* 0 -> 4*hid_channels (unet.py:112) */
